@@ -15,6 +15,7 @@ inverse Hessian) are far larger than the 126 MB L2, so nothing is flushed betwee
     python bench.py --impl reference ...                      (CPU arm: the oracle port, rank 0 only)
     python bench.py --workload cfg2|cfg3|cfg4|cfg5            (cfg2 = 8 x 1M x 1k dense; cfg4 = 8 sparse partitions
                                                                PER GPU, weak scaling; cfg5 = NaiveTrain per-key fits)
+    python bench.py --dump-outputs DIR ...                    (also write what the timed path returned in its last step)
 
 Prints ONE JSON line (rank 0).  `value` = iterations/s with inputs resident in HBM; `e2e` = the same job through
 the public API from pinned HOST buffers (upload + K iterations + model read-back in the timed region);
@@ -67,6 +68,9 @@ def parse():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--hessian-policy", type=int, default=0)
     ap.add_argument("--keys", type=int, default=100_000, help="cfg5: number of NaiveTrain keys")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step as DIR/<workload>_<name>.npy (float32 / float64, "
+                         "under 64 MB in all; see write_dump)")
     return ap.parse_args()
 
 
@@ -289,6 +293,24 @@ def log(*a):
     print("[bench]", *a, file=sys.stderr, flush=True)
 
 
+DUMP_BYTES = 60_000_000   # array data; with the .npy headers a dump stays under 64 MB
+
+
+def write_dump(path, arrays):
+    """Writes each array as path/<name>.npy so that two builds run with the same arguments can be compared output for output.
+    When the arrays exceed DUMP_BYTES together, each one is cut to its share of that budget: a sample of its elements
+    (flattened, at indices drawn with a fixed seed, in index order) that is the same from run to run."""
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for i, (name, a) in enumerate(sorted(arrays.items())):
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if total > DUMP_BYTES:
+            keep = int(a.size * DUMP_BYTES // total)
+            if keep < a.size:
+                a = a.reshape(-1)[np.sort(np.random.default_rng(i).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ GPU legs
 class Ctx:
     pass
@@ -363,6 +385,11 @@ def run_admm_workload(cx, wl, K, W, want_e2e):
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
     ms = float(tms.item())
     z_final = np.stack([sess.z(l) for l in range(L)])
+    if cx.dump is not None:
+        # what a caller of the timed job gets back: z per lambda, x and u of every (partition on this rank, lambda)
+        cx.dump[wl["name"] + "_z"] = z_final
+        cx.dump[wl["name"] + "_x"] = np.stack([np.stack([sess.x(p, l) for l in range(L)]) for p in my_parts])
+        cx.dump[wl["name"] + "_u"] = np.stack([np.stack([sess.u(p, l) for l in range(L)]) for p in my_parts])
     # size-independent invariant of the consensus step: with the unpenalised intercept z0 = mean_p(x_p + u_p), the new duals
     # u_p = float(u_p + x_p - z) sum to zero over ALL partitions (up to float rounding)
     usum = torch.tensor([[float(sess.u(p, l)[-1]) for l in range(L)] for p in my_parts], dtype=torch.float64, device=dev).sum(0)
@@ -404,6 +431,8 @@ def run_admm_workload(cx, wl, K, W, want_e2e):
         torch.cuda.synchronize()
         dt = time.perf_counter() - t0
         phases = {"upload_and_layout_s": t_up - t0, "solver_state_alloc_s": t_alloc - t_up, "iterations_and_readback_s": t0 + dt - t_alloc}
+        if cx.dump is not None:
+            cx.dump[wl["name"] + "_e2e_final_model"] = np.stack(models)
         tdt = torch.tensor([dt], dtype=torch.float64, device=dev)
         th = torch.tensor([float(h2d)], dtype=torch.float64, device=dev)
         if world > 1:
@@ -510,7 +539,8 @@ def parity_leg(cx, wl, iters=4):
 
 def run_naive_workload(cx, K, W):
     """BASELINE configs[4]: NaiveTrain per-key fits, `--keys` keys x 1000 rows x 256 dense features, lambda = 1.  Keys are
-    independent (replicas only): rank r fits keys r::N.  One "step" = one batch of 8192 keys generated on the device."""
+    independent (replicas only): rank r fits keys r::N in batches of 8192 keys generated on the device before the timed
+    region.  One "step" = one NaiveTrain job = a fit of every key of the rank."""
     import torch
     import torch.distributed as dist
     import mlease_b200 as mb
@@ -526,21 +556,18 @@ def run_naive_workload(cx, K, W):
         X = torch.randn(nkeys * nk, D, generator=g, device=dev)
         y = (torch.rand(nkeys * nk, generator=g, device=dev) < torch.sigmoid(X @ beta - 1.0)).to(torch.int32)
         return X, y, np.arange(nkeys + 1, dtype=np.int64) * nk
-    X, y, krs = batch(min(B, my_keys))
-    for _ in range(max(W, 1)):
-        mb.naive_train_dense(X, krs, y, 1.0, device=cx.local_rank, stream=stream)
+    sizes = [min(B, my_keys - k0) for k0 in range(0, my_keys, B)]
+    batches = {kb: batch(kb) for kb in dict.fromkeys(sizes)}   # full batches share one draw, the last one may be shorter
+    for X, y, krs in batches.values():
+        for _ in range(max(W, 1)):
+            mb.naive_train_dense(X, krs, y, 1.0, device=cx.local_rank, stream=stream)
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    done = 0
-    while done < my_keys:
-        kb = min(B, my_keys - done)
-        if kb != len(krs) - 1:
-            X, y, krs = batch(kb)
-        mb.naive_train_dense(X, krs, y, 1.0, device=cx.local_rank, stream=stream)
-        done += kb
+    for _ in range(K):
+        fits = [mb.naive_train_dense(batches[kb][0], batches[kb][2], batches[kb][1], 1.0, device=cx.local_rank, stream=stream) for kb in sizes]
     e1.record()
     torch.cuda.synchronize()
     tms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
@@ -548,8 +575,12 @@ def run_naive_workload(cx, K, W):
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
     if rank != 0:
         return None
+    if cx.dump is not None and K > 0:
+        # the models [keys, D+1] and skipped flags [keys] of rank 0's keys, in key order
+        cx.dump["cfg5_models"] = np.concatenate([m for m, _ in fits])
+        cx.dump["cfg5_skipped"] = np.concatenate([s for _, s in fits]).astype(np.float32)
     sec = float(tms.item()) / 1e3
-    return {"value": my_keys * world / sec, "unit": "per-key fits/s", "metric": "NaiveTrain per-key fits/sec", "seconds": sec,
+    return {"value": K * my_keys * world / sec, "unit": "per-key fits/s", "metric": "NaiveTrain per-key fits/sec", "seconds": sec,
             "keys": my_keys * world, "rows_per_key": nk, "features": D, "scaling": "weak (replicas only)"}
 
 
@@ -597,6 +628,7 @@ def main():
     cx = Ctx()
     cx.args, cx.world, cx.rank, cx.local_rank, cx.dev = args, world, rank, local_rank, "cuda:%d" % local_rank
     cx.comm = None
+    cx.dump = {} if args.dump_outputs else None
     if world > 1:
         # keep stdout to the single JSON line: NCCL's version banner / debug lines go to a file
         os.environ.setdefault("NCCL_DEBUG_FILE", "/tmp/nccl_debug_%h_%p.log")
@@ -609,6 +641,8 @@ def main():
         res = run_naive_workload(cx, K, W)
         if rank == 0:
             out.update(res)
+            if cx.dump is not None:
+                write_dump(args.dump_outputs, cx.dump)
             emit(out)
         if world > 1:
             dist.destroy_process_group()
@@ -640,6 +674,8 @@ def main():
             if world == 1 and not args.no_cpu:
                 r2["cpu_baseline"] = cpu_arm(args, wl2, K)
             out["also"][name] = r2
+    if cx.dump is not None:
+        write_dump(args.dump_outputs, cx.dump)
     emit(out)
     if world > 1:
         dist.destroy_process_group()

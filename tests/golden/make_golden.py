@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Regenerates tests/golden/*.npz.  Run HERE (container with /root/reference mounted):
+"""Regenerates the files under tests/golden/ from a checkout of the reference project (linkedin/ml-ease):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <ml-ease checkout>
 
 1. sample_data.npz   -- the reference's only fixture, examples/sample-data.avro, decoded with
                         the minimal Avro object-container reader below (null codec, Pig-style
@@ -13,6 +13,9 @@
 3. oracle_frozen.npz -- frozen outputs of oracle/mlease_oracle.cpp (exact + faithful ADMM on the
                         fixture with 4 partitions, objective values, scores, loglik) so that any
                         later edit of the oracle that changes numbers is caught.
+4. sample_data_head.avro -- the first HEAD_BLOCKS container blocks of examples/sample-data.avro, byte for
+                        byte (header, blocks, sync markers): a valid container of the file's first
+                        records, small enough to keep (the whole file is 1.26 MB).
 """
 import json
 import os
@@ -24,6 +27,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+HEAD_BLOCKS = 6
 
 
 # ----------------------------------------------------------------------------- mini avro reader
@@ -114,10 +118,32 @@ def read_avro(path):
     return schema, recs, nblocks
 
 
-def main():
+def write_sample_head(path):
+    """Copies the header and the first HEAD_BLOCKS blocks of the container at `path` to sample_data_head.avro."""
+    raw = open(path, "rb").read()
+    b = _Buf(raw)
+    assert b.raw(4) == b"Obj\x01"
+    while True:
+        n = b.long()
+        if n == 0:
+            break
+        for _ in range(abs(n)):
+            b.bytes_(), b.bytes_()
+    sync = b.raw(16)
+    for _ in range(HEAD_BLOCKS):
+        b.long()
+        b.raw(b.long())
+        assert b.raw(16) == sync
+    with open(os.path.join(HERE, "sample_data_head.avro"), "wb") as f:
+        f.write(raw[:b.i])
+
+
+def main(ref):
     from oracle import oracle as orc
 
-    schema, recs, nblocks = read_avro("/root/reference/examples/sample-data.avro")
+    src = os.path.join(ref, "examples", "sample-data.avro")
+    write_sample_head(src)
+    schema, recs, nblocks = read_avro(src)
     names = sorted({f["name"] for r in recs for f in r["features"]}, key=lambda s: int(s))
     assert all(f["term"] in ("", None) for r in recs for f in r["features"])
     gid = {n: i for i, n in enumerate(names)}
@@ -177,4 +203,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

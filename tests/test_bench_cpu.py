@@ -29,6 +29,25 @@ def test_sparse_generator_distinct_sorted_uniform_and_seeded():
     assert not np.array_equal(ci, ci3)                                                  # seed 1000 + p
 
 
+def test_dump_outputs_are_whole_within_budget_and_a_fixed_sample_beyond(tmp_path, monkeypatch):
+    import bench
+    rng = np.random.default_rng(0)
+    arrays = {"cfg3_z": rng.normal(size=(3, 101)), "cfg3_u": rng.normal(size=(2, 3, 101)).astype(np.float32)}
+    bench.write_dump(str(tmp_path / "a"), arrays)
+    for name, a in arrays.items():
+        got = np.load(str(tmp_path / "a" / (name + ".npy")))
+        assert got.dtype == a.dtype and np.array_equal(got, a)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2000)
+    for d in ("b", "c"):
+        bench.write_dump(str(tmp_path / d), arrays)
+    sizes = 0
+    for name, a in arrays.items():
+        b, c = (np.load(str(tmp_path / d / (name + ".npy"))) for d in ("b", "c"))
+        assert np.array_equal(b, c) and b.dtype == a.dtype and 0 < b.size < a.size and np.isin(b, a).all()
+        sizes += b.nbytes
+    assert sizes <= 2000
+
+
 def test_reference_arm_line_declares_its_sample():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "0",
                           "--partitions", "2", "--rows", "4000", "--features", "20000", "--cpu-rows", "1000", "--cpu-iters", "2"],
