@@ -7,8 +7,9 @@
 
 namespace mlease {
 
-constexpr int BFGS_M = 16;        // storage for secant pairs kept on top of the (possibly stale) explicit inverse Hessian
-constexpr int BFGS_M_DEFAULT = 6; // pairs actually used (Ctrl::bfgs_m)
+// secant pairs kept on top of the (possibly stale) explicit inverse Hessian.  Measured at 1M x 10k x 1 %: 12 / 16 pairs save
+// 2-4 % of the K1 passes and cost 45-60 % more two-loop time
+constexpr int BFGS_M = 6;
 
 // ------------------------------------------------------------------------------------------
 // Per-problem control block, device resident.  A "problem" is one (local partition, lambda)
@@ -29,10 +30,8 @@ struct Ctrl {
   int rejects;       // rejected trial points in this x-update
   int hess_builds;   // Gram+Cholesky rebuilds in this x-update
   int stall;         // consecutive poor contractions
-  int bfgs_count;    // secant pairs stored so far (ring of bfgs_m), reset when the Hessian is rebuilt
-  int bfgs_m;        // ring size in use (<= BFGS_M)
-  int self_scale;    // 1: adapt h0_scale from the secant pairs (set per x-update; wide systems)
-  double h0_scale;   // self-scaling factor applied to the explicit inverse inside the L-BFGS two-loop (wide systems only; 1 after a rebuild)
+  int bfgs_count;    // secant pairs stored so far (ring of BFGS_M), reset when the Hessian is rebuilt
+  double h0_scale;   // self-scaling factor applied to the explicit inverse inside the L-BFGS two-loop (rebuild_is_expensive only; 1 after a rebuild)
   int k1_chunks;     // number of per-CTA partials the last K1 pass wrote for this problem (gpart / fpart rows)
   int refresh_next;  // rebuild the Hessian at the first point of the NEXT x-update (chord steps contracted slowly)
   int skip_eval;     // 1: the gradient at the start point of this x-update is already in g_t (data term) -- see admm_consensus_kernel:
@@ -154,9 +153,6 @@ __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.p
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
   asm volatile(
@@ -223,17 +219,6 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t desc_a, uint6
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// D[tmem] (+)= A[smem desc] * B[smem desc], kind::f8f6f4 (e4m3 / e5m2 inputs, fp32 accumulate, K = 32 per instruction)
-__device__ __forceinline__ void umma_f8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // mbarrier arrive when all previously issued tcgen05.mma of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
@@ -282,6 +267,7 @@ __device__ __forceinline__ void tmem_relinquish2() { asm volatile("tcgen05.relin
 __device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t ncols) {
   asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
+// D[tmem] (+)= A[smem desc] * B[smem desc] over the pair, kind::f8f6f4 (e4m3 / e5m2 inputs, fp32 accumulate, K = 32 per instruction)
 __device__ __forceinline__ void umma_f8_2cta(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
       "{\n"

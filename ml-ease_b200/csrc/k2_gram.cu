@@ -200,18 +200,14 @@ gram_tcgen05_kernel(const Problem* __restrict__ probs, const CUtensorMap* __rest
 // ------------------------------------------------------------------------------------------
 constexpr int SK = 32;                       // data rows (K) per stage
 constexpr int S_BOX_BYTES = SK * 128;        // 4 KB = one [32 k][128 cols] e4m3 operand block
-// NCTA = 1: a CTA owns a 128 x 256 tile: A block + two B blocks per stage (12 KB), 16 stages, 8 producer trios.
-// NCTA = 2: a CTA PAIR (cluster of 2, cta_group::2) owns a 256 x 256 tile: each CTA assembles ITS 128 rows of A and ITS 128 of the
-//           B tile's 256 columns (8 KB per stage), i.e. a third less producer work, shared-memory store traffic and operand read
-//           traffic per flop; 24 stages, 12 producer pairs.  K-step k lives in stage k % SST and belongs to producer group k % NGRP
-//           (SST = 2 NGRP: a group alternates between two stages, because the refill round trip is several MMA periods long).
-template <int NCTA> struct SCfg {
-  static constexpr int SPW = NCTA == 1 ? 3 : 2;        // producer warps per stage: one per operand block
-  static constexpr int NGRP = 24 / SPW;                // producer groups
-  static constexpr int SST = 2 * NGRP;                 // ring stages
-  static constexpr int STAGE_BYTES = SPW * S_BOX_BYTES;
-  static constexpr size_t SMEM = (size_t)SST * STAGE_BYTES + 1024 /*align*/ + 512 /*barriers*/;
-};
+// A CTA PAIR (cluster of 2, cta_group::2) owns a 256 x 256 tile: each CTA assembles ITS 128 rows of A and ITS 128 of the B tile's
+// 256 columns (8 KB per stage); 24 stages, 12 producer pairs.  K-step k lives in stage k % S_SST and belongs to producer group
+// k % S_NGRP (S_SST = 2 S_NGRP: a group alternates between two stages, because the refill round trip is several MMA periods long).
+constexpr int S_SPW = 2;                       // producer warps per stage: one per operand block (A, B)
+constexpr int S_NGRP = 24 / S_SPW;             // producer groups
+constexpr int S_SST = 2 * S_NGRP;              // ring stages
+constexpr int S_STAGE_BYTES = S_SPW * S_BOX_BYTES;
+constexpr size_t S_SMEM = (size_t)S_SST * S_STAGE_BYTES + 1024 /*align*/ + 512 /*barriers*/;
 constexpr int S_THREADS = (1 + 24 + 4) * 32;   // MMA warp, 24 producer warps, 4 epilogue warps
 
 // byte offset of element (K-row k, column col < 128) inside one [32 k][128 cols] operand block of 1-byte elements: the canonical
@@ -226,19 +222,16 @@ __device__ __forceinline__ uint32_t umma_idesc_e4m3_mn(int M, int N) {
   return (1u << 4) | (1u << 15) | (1u << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
-template <int NCTA>
 __global__ void __launch_bounds__(S_THREADS, 1)
 gram_csr_tcgen05_kernel(const Problem* __restrict__ probs, const GramTile* __restrict__ tiles, int ntiles, int force, int bias_col, int share) {
-  using C = SCfg<NCTA>;
-  constexpr int SPW = C::SPW, NGRP = C::NGRP, SST = C::SST, STAGE_BYTES = C::STAGE_BYTES;
   if (share > 1 && blockIdx.z % share != 0) return;   // see gram_tcgen05_kernel (both CTAs of a pair take the same exit)
   const Problem& pb = probs[blockIdx.z];
   Ctrl* ctrl = pb.ctrl;
   if (!force && (ctrl->done || !ctrl->need_hess)) return;
-  // NCTA = 2: the tile list holds (BI, bj) of 256 x 256 tiles; this CTA's rows are the 128-block 2 BI + rank
-  const uint32_t rank = NCTA == 2 ? cluster_ctarank() : 0u;
-  const GramTile tile_in = tiles[NCTA == 2 ? (blockIdx.x >> 1) : blockIdx.x];
-  const int tile_bi = NCTA == 2 ? tile_in.bi * 2 + (int)rank : tile_in.bi;
+  // the tile list holds (BI, bj) of 256 x 256 tiles; this CTA's rows are the 128-block 2 BI + rank
+  const uint32_t rank = cluster_ctarank();
+  const GramTile tile_in = tiles[blockIdx.x >> 1];
+  const int tile_bi = tile_in.bi * 2 + (int)rank;
   const int tile_bj = tile_in.bj;
   const int slice = blockIdx.y, nslices = gridDim.y;
   const int Dp = pb.Dp;
@@ -251,71 +244,62 @@ gram_csr_tcgen05_kernel(const Problem* __restrict__ probs, const GramTile* __res
 
   extern __shared__ unsigned char g_smem_raw[];
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(g_smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + (size_t)SST * STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + SST;
-  uint64_t* acc_bar = empty_bar + SST;
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + (size_t)S_SST * S_STAGE_BYTES);
+  uint64_t* empty_bar = full_bar + S_SST;
+  uint64_t* acc_bar = empty_bar + S_SST;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_bar + 1);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   // clear the whole ring once
-  for (int e = threadIdx.x; e < SST * STAGE_BYTES / 16; e += S_THREADS) reinterpret_cast<uint4*>(smem)[e] = make_uint4(0u, 0u, 0u, 0u);
+  for (int e = threadIdx.x; e < S_SST * S_STAGE_BYTES / 16; e += S_THREADS) reinterpret_cast<uint4*>(smem)[e] = make_uint4(0u, 0u, 0u, 0u);
   if (warp == 1 && lane == 0) {
-    // full: one arrival per producer warp of the stage, of BOTH CTAs for a pair (the barrier the MMA thread waits on is the leader's)
-    for (int s = 0; s < SST; s++) { mbar_init(&full_bar[s], SPW * NCTA); mbar_init(&empty_bar[s], 1); }
+    // full: one arrival per producer warp of the stage, of BOTH CTAs (the barrier the MMA thread waits on is the leader's)
+    for (int s = 0; s < S_SST; s++) { mbar_init(&full_bar[s], S_SPW * 2); mbar_init(&empty_bar[s], 1); }
     mbar_init(acc_bar, 1);
     fence_mbar_init();
   }
-  if (warp == 0) {
-    if (NCTA == 2) { tmem_alloc2(tmem_slot, GN); tmem_relinquish2(); }
-    else { tmem_alloc(tmem_slot, GN); tmem_relinquish(); }
-  }
+  if (warp == 0) { tmem_alloc2(tmem_slot, GN); tmem_relinquish2(); }
   fence_proxy_async_smem();   // the zero fill must be visible to the async proxy too
   tc_fence_before();
-  if (NCTA == 2) cluster_sync_all(); else __syncthreads();   // the peer must see initialised barriers before its first remote arrive
+  cluster_sync_all();   // the peer must see initialised barriers before its first remote arrive
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
     if (lane == 0 && rank == 0) {
-      // ===== MMA issuer (the leader CTA's, for a pair) =====
-      // one tcgen05.mma.kind::f8f6f4 per stage: K = 32 = the stage's 32-row group (4 swizzle atoms, SBO = 1024 B apart);
-      // NCTA = 1: the B tile's second 128-column group sits LBO = 4 KB after the first; NCTA = 2: M = 256, each CTA holds one A
-      // block and one B block at the same offsets.  The loop over the ring is unrolled so that a stage's barrier addresses and
-      // descriptors are constants: at the e4m3 rate an MMA lasts ~130-220 clk, and the ~45 dependent single-thread instructions
-      // of a rolled iteration (address math, R2UR moves) were the bottleneck (ncu r02: tensor pipe 35 %).
-      const uint32_t idesc = umma_idesc_e4m3_mn(GM * NCTA, GN);
+      // ===== MMA issuer (the leader CTA's) =====
+      // one tcgen05.mma.kind::f8f6f4 per stage: K = 32 = the stage's 32-row group (4 swizzle atoms, SBO = 1024 B apart), M = 256;
+      // each CTA holds one A block and one B block at the same offsets.  The loop over the ring is unrolled so that a stage's
+      // barrier addresses and descriptors are constants: at the e4m3 rate an MMA lasts ~130-220 clk, and the ~45 dependent
+      // single-thread instructions of a rolled iteration (address math, R2UR moves) were the bottleneck (ncu r02: tensor pipe 35 %).
+      const uint32_t idesc = umma_idesc_e4m3_mn(GM * 2, GN);
       const uint32_t smem_base = smem_u32(smem);
       const uint64_t da0 = umma_desc_mn_sw128(smem_base, S_BOX_BYTES, 1024);
       const uint64_t db0 = umma_desc_mn_sw128(smem_base + S_BOX_BYTES, S_BOX_BYTES, 1024);
-      constexpr uint64_t DSTEP = (uint64_t)(STAGE_BYTES >> 4);   // the address field counts 16-byte units; the ring stays below its 14 bits
-      for (int k0 = 0; k0 < nk; k0 += SST) {
-        const uint32_t par = (uint32_t)((k0 / SST) & 1);
+      constexpr uint64_t DSTEP = (uint64_t)(S_STAGE_BYTES >> 4);   // the address field counts 16-byte units; the ring stays below its 14 bits
+      for (int k0 = 0; k0 < nk; k0 += S_SST) {
+        const uint32_t par = (uint32_t)((k0 / S_SST) & 1);
 #pragma unroll
-        for (int st = 0; st < SST; st++) {
+        for (int st = 0; st < S_SST; st++) {
           if (k0 + st < nk) {
-            if (NCTA == 2) mbar_wait_cluster(&full_bar[st], par); else mbar_wait(&full_bar[st], par);
+            mbar_wait_cluster(&full_bar[st], par);
             tc_fence_after();
-            if (NCTA == 2) {
-              umma_f8_2cta(tmem_base, da0 + (uint64_t)st * DSTEP, db0 + (uint64_t)st * DSTEP, idesc, (k0 + st) != 0 ? 1u : 0u);
-              umma_commit_2cta(&empty_bar[st]);
-            } else {
-              umma_f8(tmem_base, da0 + (uint64_t)st * DSTEP, db0 + (uint64_t)st * DSTEP, idesc, (k0 + st) != 0 ? 1u : 0u);
-              umma_commit(&empty_bar[st]);
-            }
+            umma_f8_2cta(tmem_base, da0 + (uint64_t)st * DSTEP, db0 + (uint64_t)st * DSTEP, idesc, (k0 + st) != 0 ? 1u : 0u);
+            umma_commit_2cta(&empty_bar[st]);
           }
         }
       }
-      if (NCTA == 2) umma_commit_2cta(acc_bar); else umma_commit(acc_bar);
+      umma_commit_2cta(acc_bar);
     }
   } else if (warp <= 24) {
-    // ===== producers: SPW warps per stage, one per 128-column operand block (A block; the B tile's block(s) this CTA holds).
+    // ===== producers: S_SPW warps per stage, one per 128-column operand block (the A block and the B block this CTA holds).
     // One K-step = one 32-row group, whose entries for a 128-column block are one contiguous run of the block-major list.
     // Offsets are fetched three uses ahead and the first 64 entries of a run two uses ahead, so the loads of a use are in flight
-    // during the whole previous uses.  Group t = (warp - 1) / SPW owns the K-steps k = t, t + NGRP, ...; K-step k lives in ring
-    // stage k % SST, so a group alternates between the stages t and t + NGRP.
-    const int grp = (warp - 1) / SPW, strm = (warp - 1) % SPW;
+    // during the whole previous uses.  Group t = (warp - 1) / S_SPW owns the K-steps k = t, t + S_NGRP, ...; K-step k lives in
+    // ring stage k % S_SST, so a group alternates between the stages t and t + S_NGRP.
+    const int grp = (warp - 1) / S_SPW, strm = (warp - 1) % S_SPW;
     const size_t strm_off = (size_t)strm * S_BOX_BYTES;
-    const int blk = strm == 0 ? tile_bi : (NCTA == 2 ? tile_bj * 2 + (int)rank : tile_bj * 2 + (strm - 1));
+    const int blk = strm == 0 ? tile_bi : tile_bj * 2 + (int)rank;
     const bool valid = blk < pb.nblk128;
     const long long ngroups = pb.bm_groups;
     const long long* __restrict__ my_offs = pb.bm_offs + (size_t)(valid ? blk : 0) * ngroups + (lane & 1);
@@ -327,8 +311,8 @@ gram_csr_tcgen05_kernel(const Problem* __restrict__ probs, const GramTile* __res
     const uint32_t bias_off = has_bias_col ? sw128_off(lane, bias_col - blk * 128) : 0u;
     constexpr uint32_t NOKEY = 0xFFFFFFFFu;
     const bool fetch = valid && lane < 2;
-    // the full barriers the MMA thread waits on are the leader's: a pair's producers arrive through the cluster address space
-    const uint32_t full0_remote = NCTA == 2 ? mapa_u32(&full_bar[0], 0) : 0u;
+    // the full barriers the MMA thread waits on are the leader's: the producers arrive through the cluster address space
+    const uint32_t full0_remote = mapa_u32(&full_bar[0], 0);
 
     // Pipeline registers: offsets three uses ahead (o_c), entries + sqrt(d) two uses ahead (set 2), one use ahead (set 1),
     // current (set 0); what the last TWO uses stored (p1 = previous use = the other stage, p2 = the use before = this stage).
@@ -352,19 +336,19 @@ gram_csr_tcgen05_kernel(const Problem* __restrict__ probs, const GramTile* __res
     auto to_e4m3 = [](float x) -> uint32_t { return (uint32_t)__nv_cvt_float_to_fp8(x, __NV_SATFINITE, __NV_E4M3); };
     const uint32_t smem_base_u32 = smem_u32(smem);
     {
-      const uint32_t oa = ld_offs(grp), ob = ld_offs(grp + NGRP);
+      const uint32_t oa = ld_offs(grp), ob = ld_offs(grp + S_NGRP);
       lo0 = __shfl_sync(0xffffffffu, oa, 0); hi0 = __shfl_sync(0xffffffffu, oa, 1);
       lo1 = __shfl_sync(0xffffffffu, ob, 0); hi1 = __shfl_sync(0xffffffffu, ob, 1);
     }
-    uint32_t o_c = ld_offs(grp + 2 * NGRP);
+    uint32_t o_c = ld_offs(grp + 2 * S_NGRP);
     ld_entries(lo0, hi0, key0, val0); sd0 = ld_sd(grp);
-    ld_entries(lo1, hi1, key1, val1); sd1 = ld_sd(grp + NGRP);
+    ld_entries(lo1, hi1, key1, val1); sd1 = ld_sd(grp + S_NGRP);
     bool p1row = false, p2row = false;
-    for (int k = grp, use = 0; k < nk; k += NGRP, use++) {
-      const int st = k % SST;
-      const uint32_t sbase = smem_base_u32 + (uint32_t)st * (uint32_t)STAGE_BYTES + (uint32_t)strm_off;   // shared-space address
+    for (int k = grp, use = 0; k < nk; k += S_NGRP, use++) {
+      const int st = k % S_SST;
+      const uint32_t sbase = smem_base_u32 + (uint32_t)st * (uint32_t)S_STAGE_BYTES + (uint32_t)strm_off;   // shared-space address
       // ---- un-write what the previous use of THIS STAGE (two uses ago) stored (same addresses, zero)
-      const int fill = k / SST;   // how many times this stage has been filled before
+      const int fill = k / S_SST;   // how many times this stage has been filled before
       if (fill > 0) {
         mbar_wait(&empty_bar[st], (uint32_t)((fill - 1) & 1));
 #pragma unroll
@@ -396,15 +380,13 @@ gram_csr_tcgen05_kernel(const Problem* __restrict__ probs, const GramTile* __res
       if (row_now && has_bias_col) sts_u8(sbase + bias_off, to_e4m3(sd0));
       fence_proxy_async_smem();
       __syncwarp();
-      if (lane == 0) {
-        if (NCTA == 2) mbar_arrive_cluster(full0_remote + (uint32_t)st * 8u); else mbar_arrive(&full_bar[st]);
-      }
+      if (lane == 0) mbar_arrive_cluster(full0_remote + (uint32_t)st * 8u);
       // ---- issue the loads of the use after next.  AFTER the hand-over, not before this use's stores: the fence above compiles to
       // MEMBAR.ALL.CTA, which waits for every load this thread still has in flight -- issued at the top of the use they would
       // make each hand-over wait out a DRAM round trip; issued here they have the whole next use to arrive.
       lo2 = __shfl_sync(0xffffffffu, o_c, 0); hi2 = __shfl_sync(0xffffffffu, o_c, 1);
-      o_c = ld_offs(k + 3 * NGRP);
-      ld_entries(lo2, hi2, key2, val2); sd2 = ld_sd(k + 2 * NGRP);
+      o_c = ld_offs(k + 3 * S_NGRP);
+      ld_entries(lo2, hi2, key2, val2); sd2 = ld_sd(k + 2 * S_NGRP);
       // ---- rotate
       p2lo = p1lo; p2hi = p1hi; p2row = p1row; p1lo = lo0; p1hi = hi0; p1row = row_now;
       lo0 = lo1; hi0 = hi1; lo1 = lo2; hi1 = hi2;
@@ -413,7 +395,7 @@ gram_csr_tcgen05_kernel(const Problem* __restrict__ probs, const GramTile* __res
       sd0 = sd1; sd1 = sd2;
     }
   } else {
-    // ===== epilogue: the last four warps -> TMEM lane quadrant (warp % 4); a pair's CTA holds its own 128 rows of the tile =====
+    // ===== epilogue: the last four warps -> TMEM lane quadrant (warp % 4); each CTA of the pair holds its own 128 rows of the tile =====
     const int quad = warp & 3;
     float* out = pb.Hpart + (size_t)slice * Dp * Dp;
     const int row = tile_bi * GM + quad * 32 + lane;
@@ -442,19 +424,11 @@ gram_csr_tcgen05_kernel(const Problem* __restrict__ probs, const GramTile* __res
     }
     tc_fence_before();
   }
-  if (NCTA == 2) {
-    tc_fence_before();
-    cluster_sync_all();   // neither CTA may leave (or free its TMEM) while the pair's MMAs, commits or remote arrives can still touch it
-    if (warp == 0) {
-      tc_fence_after();
-      tmem_dealloc2(tmem_base, GN);
-    }
-  } else {
-    __syncthreads();
-    if (warp == 0) {
-      tc_fence_after();
-      tmem_dealloc(tmem_base, GN);
-    }
+  tc_fence_before();
+  cluster_sync_all();   // neither CTA may leave (or free its TMEM) while the pair's MMAs, commits or remote arrives can still touch it
+  if (warp == 0) {
+    tc_fence_after();
+    tmem_dealloc2(tmem_base, GN);
   }
 }
 
@@ -614,43 +588,31 @@ cudaError_t gram_launch_tcgen05(const Problem* d_probs, int nprob, const void* d
   return cudaGetLastError();
 }
 
-template <int NCTA>
-static cudaError_t gram_csr_configure() {
-  // the attribute is per device: set it once for every device this process launches on
-  static bool configured[64] = {};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64 || !configured[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(gram_csr_tcgen05_kernel<NCTA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SCfg<NCTA>::SMEM);
-    if (e != cudaSuccess) return e;
-    if (dev >= 0 && dev < 64) configured[dev] = true;
-  }
-  return cudaSuccess;
-}
-
-// ncta = 2: d_tiles holds 256 x 256 pair tiles (gram_tile_list(..., 1)); the grid is a list of 2-CTA clusters along x.
+// d_tiles holds 256 x 256 pair tiles (gram_tile_list(..., 1)); the grid is a list of 2-CTA clusters along x.
 cudaError_t gram_launch_csr_tcgen05(const Problem* d_probs, int nprob, const void* d_tiles, int ntiles, int nslices, int force,
-                                    int bias_col, cudaStream_t st, int* launches, int share, int ncta) {
-  const GramTile* tl = reinterpret_cast<const GramTile*>(d_tiles);
-  if (ncta == 2) {
-    cudaError_t e = gram_csr_configure<2>();
-    if (e != cudaSuccess) return e;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * ntiles, nslices, nprob);
-    cfg.blockDim = dim3(S_THREADS, 1, 1);
-    cfg.dynamicSmemBytes = SCfg<2>::SMEM;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    e = cudaLaunchKernelEx(&cfg, gram_csr_tcgen05_kernel<2>, d_probs, tl, ntiles, force, bias_col, share);
-    if (e != cudaSuccess) return e;
-  } else {
-    cudaError_t e = gram_csr_configure<1>();
-    if (e != cudaSuccess) return e;
-    gram_csr_tcgen05_kernel<1><<<dim3(ntiles, nslices, nprob), S_THREADS, SCfg<1>::SMEM, st>>>(d_probs, tl, ntiles, force, bias_col, share);
+                                    int bias_col, cudaStream_t st, int* launches, int share) {
+  {
+    // the attribute is per device: set it once for every device this process launches on
+    static bool configured[64] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64 || !configured[dev]) {
+      cudaError_t e = cudaFuncSetAttribute(gram_csr_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S_SMEM);
+      if (e != cudaSuccess) return e;
+      if (dev >= 0 && dev < 64) configured[dev] = true;
+    }
   }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(2 * ntiles, nslices, nprob);
+  cfg.blockDim = dim3(S_THREADS, 1, 1);
+  cfg.dynamicSmemBytes = S_SMEM;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, gram_csr_tcgen05_kernel, d_probs, reinterpret_cast<const GramTile*>(d_tiles), ntiles, force, bias_col, share);
+  if (e != cudaSuccess) return e;
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

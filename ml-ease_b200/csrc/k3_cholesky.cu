@@ -9,7 +9,6 @@
 // break down when cond(H) approaches 1/eps_fp32; 3.3e8 flop at D'=1001 is latency- not
 // throughput-bound on B200's fp64 pipe.
 #include <algorithm>
-#include <cstdlib>
 
 #include "kernels.cuh"
 
@@ -528,7 +527,6 @@ static cudaError_t dgemm_launch(const Problem* d_probs, int nprob, int mode, int
 // Shared-memory strides: A rows of 20 words (fragment loads (row g, k tg): bank 20 g + tg, all distinct), B rows of 136
 // words (fragment loads (k tg, col g): bank 8 tg + g, all distinct).
 // ------------------------------------------------------------------------------------------
-constexpr int MERGE_TF32_DEFAULT = 1;   // verified on a B200: GPU parity suite + bench with MLEASE_MERGE_TF32=1 (profiles/r02b_*)
 constexpr int TM = 128, TN = 128, TK = 16;
 constexpr int TA_LD = TK + 4, TB_LD = TN + 8;
 constexpr int TA_SZ = TM * TA_LD, TB_SZ = TK * TB_LD;   // 32-bit words per stage
@@ -682,25 +680,9 @@ static cudaError_t merge_tf32_launch(const Problem* d_probs, int nprob, int mode
   if (launches) *launches += 1;
   return cudaGetLastError();
 }
-// MLEASE_MERGE_TF32=0 / 1 selects the fp64 DMMA merges / the TF32 merges (A/B measurements); see the default below.
-static bool merges_in_tf32() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MLEASE_MERGE_TF32");
-    v = e ? (atoi(e) ? 1 : 0) : MERGE_TF32_DEFAULT;
-  }
-  return v == 1;
-}
-
-// Systems wider than this take the GEMM-rich path.  MLEASE_WIDE_MIN overrides it (tuning experiments only).
-static int wide_threshold() {
-  static int t = -1;
-  if (t < 0) {
-    const char* e = getenv("MLEASE_WIDE_MIN");
-    t = e ? atoi(e) : 1000;   // measured on B200: D'=1001 (ldh 1024) rebuilds take 4.9 ms (8 problems) / 2.0 ms (1) wide vs 8.1 / 2.75 ms narrow
-  }
-  return t;
-}
+// Systems wider than this take the GEMM-rich path.
+// Measured on B200: D'=1001 (ldh 1024) rebuilds take 4.9 ms (8 problems) / 2.0 ms (1) wide vs 8.1 / 2.75 ms narrow.
+constexpr int WIDE_MIN = 1000;
 
 // Wide systems (Ysym != NULL, ldh > 2048): the solver never needs H^-1 itself, only the
 // product H^-1 q = Y^T (Y q) with Y = L^-1.  Ysym receives Y (bf16) in SYMMETRIC storage, M[i][j] = Y[max(i,j)][min(i,j)]: row r of
@@ -729,7 +711,7 @@ __global__ void __launch_bounds__(256) ysym_kernel(const Problem* __restrict__ p
   }
 }
 
-bool cholesky_factored_direction(int ldh) { return ldh > 2048 && ldh > wide_threshold(); }   // = the problems that carry Ysym (batch_alloc)
+bool cholesky_factored_direction(int ldh) { return ldh > 2048; }   // = the problems that carry Ysym (batch_alloc)
 
 static cudaError_t cholesky_launch_wide(const Problem* d_probs, int nprob, int ldh, cudaStream_t st, int* launches, bool factored_direction) {
   cudaError_t e;
@@ -757,10 +739,9 @@ static cudaError_t cholesky_launch_wide(const Problem* d_probs, int nprob, int l
   if (launches) *launches += 1;
   // the factored direction reads Y only as bf16 (ysym_kernel): its merges run in TF32; an explicit H^-1 (posterior variance,
   // systems up to 2048 columns) keeps the fp64 merges
-  const bool tf32 = factored_direction && merges_in_tf32();
   for (int m = WLEAF; m < ldh; m *= 2) {
     const int nmerge = (ldh + 2 * m - 1) / (2 * m);
-    if (tf32) {
+    if (factored_direction) {
       if ((e = merge_tf32_launch(d_probs, nprob, 1, m, nmerge, st, launches)) != cudaSuccess) return e;
       if ((e = merge_tf32_launch(d_probs, nprob, 2, m, nmerge, st, launches)) != cudaSuccess) return e;
       continue;
@@ -818,7 +799,7 @@ cudaError_t cholesky_launch(const Problem* d_probs, int nprob, int ldh, cudaStre
     if (launches) *launches += 1;
   }
   const int nb = ldh / NB;
-  if (ldh > wide_threshold()) {
+  if (ldh > WIDE_MIN) {
     cudaError_t e = cholesky_launch_wide(d_probs, nprob, ldh, st, launches, cholesky_factored_direction(ldh) && !want_hinv);
     if (e != cudaSuccess) return e;
   } else {

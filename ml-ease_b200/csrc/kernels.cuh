@@ -19,7 +19,7 @@ cudaError_t k1f_launch(const Problem* d_probs, int ngroups, int L, int S, int LP
 
 // Newton state machine (newton.cu)
 cudaError_t newton_begin(const Problem* d_probs, int nprob, double xtol, int max_newton, int hess_policy,
-                         int invalidate_hess, int rebuild_is_expensive, cudaStream_t st, int* launches, int bfgs_m = BFGS_M_DEFAULT, int self_scale = 0);
+                         int invalidate_hess, int rebuild_is_expensive, cudaStream_t st, int* launches);
 cudaError_t k1_reduce_decide(const Problem* d_probs, int nprob, int Dt, cudaStream_t st, int* launches, int spec = 0);
 cudaError_t newton_solve(const Problem* d_probs, int nprob, int ldh, cudaStream_t st, int* launches, int group_L = 1);
 
@@ -29,7 +29,7 @@ int gram_tile_list(int Dp, short* bi_bj_pairs, int max_tiles, int pair_tiles = 0
 cudaError_t gram_launch_tcgen05(const Problem* d_probs, int nprob, const void* d_tmaps, const void* d_tiles, int ntiles,
                                 int nslices, int force, cudaStream_t st, int* launches, int share = 0);
 cudaError_t gram_launch_csr_tcgen05(const Problem* d_probs, int nprob, const void* d_tiles, int ntiles, int nslices, int force,
-                                    int bias_col, cudaStream_t st, int* launches, int share = 0, int ncta = 1);
+                                    int bias_col, cudaStream_t st, int* launches, int share = 0);
 cudaError_t csr_bm_offsets(long long n, const long long* rowptr, const int* colidx, int nblk, long long ngroups, long long* offs, cudaStream_t st);
 cudaError_t csr_bm_fill(long long n, const long long* rowptr, const int* colidx, const float* vals, int nblk, long long ngroups,
                         const long long* offs, unsigned short* keys, float* bvals, cudaStream_t st);

@@ -37,7 +37,7 @@ __device__ __forceinline__ double block_max(double v, double* sc) {
 // Start of an x-update: beta = beta_t = init, flags reset.  init/m/q were written by the caller
 // (ADMM consensus kernel or mlease_fit_partition).
 __global__ void newton_begin_kernel(const Problem* __restrict__ probs, double xtol, int max_newton, int hess_policy,
-                                    int invalidate_hess, int rebuild_is_expensive, int bfgs_m, int self_scale) {
+                                    int invalidate_hess, int rebuild_is_expensive) {
   const Problem& pb = probs[blockIdx.x];
   Ctrl* c = pb.ctrl;
   for (int k = threadIdx.x; k < pb.ldx; k += blockDim.x) {
@@ -58,9 +58,7 @@ __global__ void newton_begin_kernel(const Problem* __restrict__ probs, double xt
     c->newton_steps = 0; c->evals = 0; c->rejects = 0; c->hess_builds = 0; c->stall = 0; c->build_step = 0; c->warm_used = 0;
     c->alpha = 1.0; c->phi0 = 0.0; c->f_acc = 0.0; c->f_t = 0.0; c->gnorm = 0.0; c->gnorm_prev = 0.0; c->dirnorm = 0.0; c->dirnorm_prev = 0.0;
     c->xtol = xtol; c->max_newton = max_newton; c->hess_policy = hess_policy; c->rebuild_is_expensive = rebuild_is_expensive;
-    if (c->bfgs_m != bfgs_m) { c->bfgs_m = bfgs_m; c->bfgs_count = 0; }
-    c->self_scale = self_scale;
-    if (!self_scale) c->h0_scale = 1.0;
+    if (!rebuild_is_expensive) c->h0_scale = 1.0;
     // Rebuild at the start point when there is no factor, when the policy says always, or when the previous
     // x-update's chord steps contracted slowly: a factor taken at a (nearly) converged point makes every later
     // x-update of the ADMM run a 2-3 pass affair, and costs about as much as 2.5 K1 passes.
@@ -207,14 +205,14 @@ __global__ void __launch_bounds__(1024) k1_reduce_decide_kernel(const Problem* _
     // below runs), so that both loops of the recursion see the same, empty, pair set.
     if (action == 1 && c->need_hess) c->bfgs_count = 0;
     if (action == 1 && have_dir && !c->need_hess && sy > 1e-10 * sqrt(ss * yy2) && sy > 0.0) {   // strictly convex => s.y > 0 up to rounding
-      s_slot = c->bfgs_count % c->bfgs_m;
+      s_slot = c->bfgs_count % BFGS_M;
       pb.bfgs_rho[s_slot] = 1.0 / sy;
       c->bfgs_count++;
       // Self-scaling of the stale inverse (systems too wide to refactorise mid-run keep the factor of the cold start, where
       // every IRLS weight is at its maximum 1/4: H0 is uniformly too small an inverse).  Along the accepted step the model
       // predicted a gradient change of -alpha*phi0, the data returned s.y: their ratio is how much longer the step should
       // have been.  Standard L-BFGS practice (gamma = s.y / y.y for H0 = I), taken along s so that it costs no extra GEMV.
-      if (c->self_scale) {
+      if (c->rebuild_is_expensive) {
         const double tau = fmin(fmax(-(alpha * c->phi0) / sy, 0.5), 2.0);
         c->h0_scale = fmin(fmax(c->h0_scale * tau, 0.25), 16.0);
       }
@@ -246,12 +244,12 @@ __global__ void __launch_bounds__(1024) k1_reduce_decide_kernel(const Problem* _
   __syncthreads();
   if (c->done || !c->need_solve) return;
   {
-    const int npairs = min(c->bfgs_count, c->bfgs_m);
+    const int npairs = min(c->bfgs_count, BFGS_M);
     double* q = pb.g_t;   // free scratch from here until the next K1 reduce
     for (int k = threadIdx.x; k < Dt; k += NTD) q[k] = pb.g_acc[k];
     __syncthreads();
     for (int j = 0; j < npairs; j++) {
-      const int slot = (c->bfgs_count - 1 - j) % c->bfgs_m;
+      const int slot = (c->bfgs_count - 1 - j) % BFGS_M;
       const double* S = pb.bfgs_S + (size_t)slot * ldx;
       const double* Y = pb.bfgs_Y + (size_t)slot * ldx;
       double d = 0.0;
@@ -410,14 +408,14 @@ __global__ void __launch_bounds__(1024) newton_solve_kernel(const Problem* __res
   const int Dt = pb.Dt, ldx = pb.ldx;
   double* rhs = pb.dir;
   {
-    const int npairs = min(c->bfgs_count, c->bfgs_m);
+    const int npairs = min(c->bfgs_count, BFGS_M);
     const double h0s = c->h0_scale;
     if (h0s != 1.0) {
       for (int k = tid; k < Dt; k += NTD) rhs[k] *= h0s;
       __syncthreads();
     }
     for (int j = npairs - 1; j >= 0; j--) {
-      const int slot = (c->bfgs_count - 1 - j) % c->bfgs_m;
+      const int slot = (c->bfgs_count - 1 - j) % BFGS_M;
       const double* S = pb.bfgs_S + (size_t)slot * ldx;
       const double* Y = pb.bfgs_Y + (size_t)slot * ldx;
       double d = 0.0;
@@ -475,9 +473,8 @@ __global__ void __launch_bounds__(1024) newton_solve_kernel(const Problem* __res
 }
 
 cudaError_t newton_begin(const Problem* d_probs, int nprob, double xtol, int max_newton, int hess_policy,
-                         int invalidate_hess, int rebuild_is_expensive, cudaStream_t st, int* launches, int bfgs_m, int self_scale) {
-  newton_begin_kernel<<<nprob, 256, 0, st>>>(d_probs, xtol, max_newton, hess_policy, invalidate_hess, rebuild_is_expensive,
-                                             bfgs_m < 1 ? 1 : (bfgs_m > BFGS_M ? BFGS_M : bfgs_m), self_scale);
+                         int invalidate_hess, int rebuild_is_expensive, cudaStream_t st, int* launches) {
+  newton_begin_kernel<<<nprob, 256, 0, st>>>(d_probs, xtol, max_newton, hess_policy, invalidate_hess, rebuild_is_expensive);
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

@@ -143,16 +143,15 @@ struct Batch {
   bool csr = false;
   int has_bias = 1;
   int k1_grid = 1, gram_slices = 1, ntiles = 0;
-  int gram_ncta = 1;              // 2: the CSR Gram runs on CTA pairs (cta_group::2, 256 x 256 tiles); d_tiles then holds pair tiles
-  int gram_from_csr = 0;          // every problem of the batch assembles its Gram tiles from CSR (no dense bf16 operand)
+  int gram_from_csr = 0;          // every problem of the batch assembles its Gram tiles from CSR (no dense bf16 operand) on CTA
+                                  // pairs (cta_group::2, 256 x 256 tiles); d_tiles then holds pair tiles
   int group_L = 1;                // problems b = g * group_L + l share the data of partition g (the lambdas of one partition)
   int k1_fused = 0;               // the fused multi-lambda CSR K1 runs (segment lists present): one launch, grid (sg_S, nprob / group_L)
   int k1f_LP = 1;                 // lambdas padded to 1 / 2 / 4 in the interleaved shared-memory vectors
   size_t k1f_smem = 0;
   int k1_dyn = 0;                 // > 0: K1 CTAs are dealt to the running problems at run time (value = nprob, <= 32); k1_grid = whole grid
-  int self_scale = 0;             // adapt a scalar multiplier of the stale inverse from the secant pairs (wide systems)
-  int bfgs_m = BFGS_M_DEFAULT;    // secant pairs in use
-  int rebuild_is_expensive = 0;   // cost model: Gram + Cholesky + inverse vs one K1 pass (set in batch_alloc)
+  int rebuild_is_expensive = 0;   // cost model: Gram + Cholesky + inverse vs one K1 pass (set in batch_alloc); also turns on the
+                                  // self-scaling of the stale inverse from the secant pairs
   std::vector<Problem> h;
   Problem* d = nullptr;
   Problem* d_compact = nullptr;   // large batches: Problem structs of the problems that may rebuild in the next slot
@@ -245,7 +244,7 @@ int batch_alloc(Batch& B, int num_sms) {
   for (auto& p : B.h) if (!p.bm_offs) B.gram_from_csr = 0;
   // fused multi-lambda CSR K1: every problem has segment lists, the groups are whole, and the shared-memory vectors fit
   B.k1_fused = 0;
-  if (B.csr && B.gram_from_csr && B.group_L >= 1 && B.group_L <= 4 && nprob % B.group_L == 0 && !getenv("MLEASE_NO_FUSED_K1")) {
+  if (B.csr && B.gram_from_csr && B.group_L >= 1 && B.group_L <= 4 && nprob % B.group_L == 0) {
     bool ok = true;
     for (auto& p : B.h) if (!p.sg_perm || p.sg_S != B.h[0].sg_S || p.sg_rows != B.h[0].sg_rows) ok = false;
     if (ok) {
@@ -265,21 +264,16 @@ int batch_alloc(Batch& B, int num_sms) {
     // only wide systems qualify: small ones (NaiveTrain's per-key fits, cold-started every time) are launch-bound, not
     // flop-bound, and a mid-update rebuild saves them many lock-step slots
     B.rebuild_is_expensive = (t_rebuild > 8.0 * t_pass && B.Dt > 2048) ? 1 : 0;
-    B.self_scale = B.rebuild_is_expensive;
-    if (const char* e = getenv("MLEASE_SELF_SCALE")) B.self_scale = atoi(e) ? 1 : 0;   // tuning experiments only
-    B.bfgs_m = BFGS_M_DEFAULT;   // measured at 1M x 10k x 1 %: 12 / 16 pairs save 2-4 % of the K1 passes and cost 45-60 % more two-loop time
-    if (const char* e = getenv("MLEASE_BFGS_M")) B.bfgs_m = std::max(1, std::min(BFGS_M, atoi(e)));   // tuning experiments only
   }
   // Gram decomposition
   constexpr int MAX_TILES = 1 << 18;   // lower 128x256 tiles of Dp up to ~90k
   std::vector<short> tiles(2 * (size_t)MAX_TILES);
-  B.gram_ncta = (B.gram_from_csr && !getenv("MLEASE_GRAM_1CTA")) ? 2 : 1;   // the variable exists for A/B measurements only
-  B.ntiles = gram_tile_list(B.Dp, tiles.data(), MAX_TILES, B.gram_ncta == 2);
+  B.ntiles = gram_tile_list(B.Dp, tiles.data(), MAX_TILES, B.gram_from_csr);
   if (B.ntiles <= 0) return fail(MLEASE_ERR_INVALID, "Gram tile list overflow");
   {
     const long long ksteps = (maxn + 63) / 64;
     const long long base = (long long)B.ntiles * nprob;   // CTAs, or CTA pairs
-    const long long cap = std::max(1, num_sms / B.gram_ncta);
+    const long long cap = std::max(1, num_sms / (B.gram_from_csr ? 2 : 1));
     int best = 1;
     double best_eff = 0;
     for (int s = 1; s <= 16; s++) {
@@ -308,7 +302,7 @@ int batch_alloc(Batch& B, int num_sms) {
   if (int rc = dev_alloc(B, (void**)&yi, (size_t)nprob * B.ldh * B.ldh * sizeof(double))) return rc;
   if (int rc = dev_alloc(B, (void**)&hi, (size_t)nprob * B.ldh * B.ldh * sizeof(double))) return rc;
   __nv_bfloat16* hif = nullptr;
-  if (B.ldh > 2048)
+  if (cholesky_factored_direction(B.ldh))
     if (int rc = dev_alloc(B, (void**)&hif, (size_t)nprob * B.ldh * B.ldh * sizeof(__nv_bfloat16))) return rc;
   if (int rc = dev_alloc(B, (void**)&B.d_ctrl, (size_t)nprob * sizeof(Ctrl))) return rc;
   if (int rc = dev_alloc(B, (void**)&B.d, (size_t)nprob * sizeof(Problem))) return rc;
@@ -379,13 +373,20 @@ cudaError_t batch_k1(Batch& B, int force_emit, cudaStream_t st, int* launches) {
   return k1_launch(B.d, B.nprob, B.csr, B.ldx, B.has_bias, B.k1_grid, force_emit, st, launches, B.gram_from_csr, B.k1_dyn);
 }
 
+// Gram of a rebuild over d_probs (B.d or its compacted copy): operand tiles assembled from CSR on CTA pairs, or the dense TMA kernel
+cudaError_t batch_gram(Batch& B, const Problem* d_probs, int nprob, int force, int share, cudaStream_t st, int* launches) {
+  if (B.gram_from_csr)
+    return gram_launch_csr_tcgen05(d_probs, nprob, B.d_tiles, B.ntiles, B.gram_slices, force, B.has_bias ? B.Dt - 1 : -1, st, launches, share);
+  return gram_launch_tcgen05(d_probs, nprob, B.d_tmaps, B.d_tiles, B.ntiles, B.gram_slices, force, st, launches, share);
+}
+
 // One x-update for every problem of the batch: beta (init), m, q must already be on the device.
 int batch_xupdate(Batch& B, cudaStream_t st, double xtol, int max_newton, int policy, int invalidate, int* h_flag, int* d_flag,
                   Counters& cnt, Profiler* prof = nullptr, int share_first_gram = 0, int share_first_factor = 0) {
   Profiler nop;
   Profiler& pf = prof ? *prof : nop;
   int launches = 0;
-  CK(newton_begin(B.d, B.nprob, xtol, max_newton, policy, invalidate, B.rebuild_is_expensive, st, &launches, B.bfgs_m, B.self_scale));
+  CK(newton_begin(B.d, B.nprob, xtol, max_newton, policy, invalidate, B.rebuild_is_expensive, st, &launches));
   // The first slot's flags are known on the host: every problem is running, and a rebuild is due iff the policy says
   // always, the factors were invalidated, or the mirrored control blocks say so (no factor yet / refresh requested).
   const bool small = B.nprob <= 64;   // small batches read the whole control array back each slot (one sync, no poll kernel)
@@ -415,8 +416,7 @@ int batch_xupdate(Batch& B, cudaStream_t st, double xtol, int max_newton, int po
       const int share = (slot_idx == 0) ? share_first_gram : 0;
       if (share > 1)
         for (int b = 0; b < B.nprob; b++) if (b % share != 0) shared_flops += (double)B.h[b].n * (double)B.Dt * (double)(B.Dt + 1);
-      if (B.gram_from_csr) CK(gram_launch_csr_tcgen05(d_hess, n_hess, B.d_tiles, B.ntiles, B.gram_slices, 0, B.has_bias ? B.Dt - 1 : -1, st, &launches, share, B.gram_ncta));
-      else CK(gram_launch_tcgen05(d_hess, n_hess, B.d_tmaps, B.d_tiles, B.ntiles, B.gram_slices, 0, st, &launches, share));
+      CK(batch_gram(B, d_hess, n_hess, 0, share, st, &launches));
       pf.end(st);
       pf.begin(3, st);
       const bool share_fact = share > 1 && share_first_factor;   // same rho too: same H, one factorisation per group
@@ -451,7 +451,7 @@ int batch_xupdate(Batch& B, cudaStream_t st, double xtol, int max_newton, int po
       if (!B.h_ctrl[i]) CK(cudaMallocHost((void**)&B.h_ctrl[i], (size_t)B.nprob * sizeof(Ctrl)));
       if (!B.slot_ev[i]) CK(cudaEventCreateWithFlags(&B.slot_ev[i], cudaEventDisableTiming));
     }
-    const bool may_spec = policy == 0 && !getenv("MLEASE_NO_SLOT_PIPELINE");
+    const bool may_spec = policy == 0;
     auto flags_of = [&](const Ctrl* c, bool* all_valid) {
       int f = 0; bool v = true;
       for (int b = 0; b < B.nprob; b++) if (!c[b].done) { f |= 1; if (c[b].emit) f |= 2; if (!c[b].hess_valid) v = false; }
@@ -948,7 +948,9 @@ static int csr_build_layout(mlease_session* s, PartData& pd) {
     CK(csr_bm_offsets(nrows, pd.rowptr, pd.colidx, pd.nblk128, pd.bm_groups, (long long*)bo, s->stream));
     CK(csr_bm_fill(nrows, pd.rowptr, pd.colidx, pd.vals, pd.nblk128, pd.bm_groups, (const long long*)bo, (unsigned short*)bk, (float*)bv, s->stream));
     pd.bm_offs = (long long*)bo; pd.bm_keys = (unsigned short*)bk; pd.bm_vals = (float*)bv;
-    // segment lists of the fused multi-lambda K1
+    // segment lists of the fused multi-lambda K1.  MLEASE_NO_FUSED_K1 is a test hook: without the lists batch_alloc falls back to
+    // the per-problem CSR kernels, which production runs for NaiveTrain, for more than 4 lambdas and when the fused kernel's
+    // shared memory overflows; the hook lets the tests reach them on small inputs
     int S = 0, rows = 0, LP = 0; size_t smem = 0;
     if (!getenv("MLEASE_NO_FUSED_K1") && k1f_plan(nrows, s->ldx, s->L, s->num_sms, &S, &rows, &LP, &smem)) {
       CK(k1f_build(nrows, s->Dg, pd.nnz, pd.rowptr, pd.colidx, pd.vals, S, rows, &pd.sg_ngrp, &pd.sg_perm, &pd.sg_depth, &pd.sg_goff, &pd.sg_row16,
@@ -1283,8 +1285,7 @@ int mlease_objective(mlease_session* s, int32_t pid, const double* w, const doub
   if (f) *f = c.f_t;
   if (H) {
     if (!tensor && B->gram_from_csr) return fail(MLEASE_ERR_INVALID, "the SIMT debug Gram needs the dense bf16 operand, which CSR partitions with sorted unique rows do not materialise");
-    if (tensor && B->gram_from_csr) CK(gram_launch_csr_tcgen05(B->d, 1, B->d_tiles, B->ntiles, B->gram_slices, 1, B->has_bias ? B->Dt - 1 : -1, s->stream, &launches, 0, B->gram_ncta));
-    else if (tensor) CK(gram_launch_tcgen05(B->d, 1, B->d_tmaps, B->d_tiles, B->ntiles, B->gram_slices, 1, s->stream, &launches));
+    if (tensor) CK(batch_gram(*B, B->d, 1, 1, 0, s->stream, &launches));
     else CK(gram_launch_simt(B->d, 1, B->Dp, 1, s->stream, &launches));
     if (tensor == 2) {
       // the inverse the Newton direction uses: split-K Gram partials + diag(q) -> fp64 Cholesky -> explicit inverse
@@ -1403,10 +1404,8 @@ int mlease_time_kernel(mlease_session* s, int32_t pid, int32_t which, int32_t re
   CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
   // warm-up launch (also produces the scaled copy the Gram needs)
   CK(batch_k1(*B, 1, s->stream, &launches));
-  const int bias_col = B->has_bias ? B->Dt - 1 : -1;
   if (which == 3) {
-    if (B->gram_from_csr) CK(gram_launch_csr_tcgen05(B->d, 1, B->d_tiles, B->ntiles, B->gram_slices, 1, bias_col, s->stream, &launches, 0, B->gram_ncta));
-    else CK(gram_launch_tcgen05(B->d, 1, B->d_tmaps, B->d_tiles, B->ntiles, B->gram_slices, 1, s->stream, &launches));
+    CK(batch_gram(*B, B->d, 1, 1, 0, s->stream, &launches));
     Ctrl c; std::memset(&c, 0, sizeof(c)); c.need_hess = 1;
     CK(cudaMemcpyAsync(B->d_ctrl, &c, sizeof(Ctrl), cudaMemcpyHostToDevice, s->stream));
   }
@@ -1414,8 +1413,7 @@ int mlease_time_kernel(mlease_session* s, int32_t pid, int32_t which, int32_t re
   CK(cudaEventRecord(e0, s->stream));
   for (int r = 0; r < reps; r++) {
     if (which == 1) CK(batch_k1(*B, emit_scaled ? 1 : 0, s->stream, &launches));
-    else if (which == 2 && B->gram_from_csr) CK(gram_launch_csr_tcgen05(B->d, 1, B->d_tiles, B->ntiles, B->gram_slices, 1, bias_col, s->stream, &launches, 0, B->gram_ncta));
-    else if (which == 2) CK(gram_launch_tcgen05(B->d, 1, B->d_tmaps, B->d_tiles, B->ntiles, B->gram_slices, 1, s->stream, &launches));
+    else if (which == 2) CK(batch_gram(*B, B->d, 1, 1, 0, s->stream, &launches));
     else if (which == 3) CK(cholesky_launch(B->d, 1, B->ldh, s->stream, &launches));
     else return fail(MLEASE_ERR_INVALID, "which must be 1, 2 or 3");
   }

@@ -63,6 +63,17 @@ def test_product_package_never_imports_the_oracle():
                 assert not bad.search(txt), os.path.join(dp, f)
 
 
+def test_device_library_reads_only_known_environment_variables():
+    """The device library takes no tuning switches from the environment: one test hook (segment lists off, so the per-problem
+    CSR K1 kernels run) and two diagnostics that only print.  A code path selected by an environment variable is a path
+    that neither the tests nor the benchmark run."""
+    csrc = os.path.join(ROOT, "ml-ease_b200", "csrc")
+    names = set()
+    for f in os.listdir(csrc):
+        names |= set(re.findall(r'getenv\(\s*"([^"]+)"', open(os.path.join(csrc, f)).read()))
+    assert names == {"MLEASE_NO_FUSED_K1", "MLEASE_DEBUG", "MLEASE_UPLOAD_TRACE"}, sorted(names)
+
+
 def test_tools_and_bench_scripts_parse():
     """The GPU-side scripts cannot run here, but they must at least be valid Python and bench.py must keep its CLI contract."""
     import ast
